@@ -26,6 +26,7 @@
 
 Launch:  python bench.py --gpus 1 --steps K --warmup W          (N>1: via torch.distributed.run, one rank per GPU)
          python bench.py --impl reference ...                   (the reference arm: CPU implementation of the path)
+         python bench.py ... --dump-outputs DIR                 (also write what the last timed step computed, see dump_outputs)
 """
 import argparse
 import ctypes
@@ -34,6 +35,7 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -181,6 +183,37 @@ def vkfft_cuda_reference(torch, buf, ns, iters=5, warm=2):
         out["sample0_style_score"] = sum(score_terms) / len(score_terms)
     return out
 
+
+
+DUMP_POINTS = 1 << 17                # points of the buffer written per array by --dump-outputs (1 MiB of complex64)
+
+
+def dump_outputs(out_dir, torch, vk, apps, lp, buf, start, steps, sweep):
+    """--dump-outputs: what the timed steps' last step computed, as a caller of each VkFFTAppend receives it in `buf`, written
+    as DIR/<name>.npy float32 arrays [DUMP_POINTS, 2] (re, im) at one fixed, seeded sample of buffer positions:
+      input                the buffer as the last step received it
+      forward_n<N>, inverse_n<N>   the buffer after that step's forward / inverse transform of length N (in sweep order)
+    The step is replayed from `start` (a copy of the buffer taken just before the timed steps) after the same number of sweeps;
+    the replay must reproduce the timed steps' result bit for bit at the sampled positions, or nothing is written."""
+    import numpy as np
+    idx = np.sort(np.random.default_rng(0).choice(buf.numel(), DUMP_POINTS, replace=False))
+    idx = torch.from_numpy(idx).to(buf.device)
+    timed = buf[idx]
+    buf.copy_(start)
+    for _ in range(steps - 1):
+        sweep()
+    arrays = {"input": buf[idx]}
+    for n, app, _ in apps:
+        for inv, name in ((-1, "forward"), (1, "inverse")):
+            rc = vk.VkFFTAppend(app, inv, lp)
+            if rc:
+                raise RuntimeError(vk.getVkFFTErrorString(rc))
+            arrays[f"{name}_n{n}"] = buf[idx]
+    assert torch.equal(buf[idx], timed), "the replayed step differs from the timed one"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), torch.view_as_real(a).cpu().numpy())
+    return {"dir": out_dir, "arrays": len(arrays), "points_per_array": DUMP_POINTS, "dtype": "float32 (re, im)"}
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -385,8 +418,9 @@ def sample0_scores(device_index):
             continue
         try:
             t0 = time.time()
-            r = subprocess.run([path, "-d", str(device_index), "-vkfft", "0"], capture_output=True, text=True, timeout=900,
-                               cwd=os.path.join(ROOT, "oracle", "_ref"))
+            with tempfile.TemporaryDirectory() as td:      # the program writes its kernel cache to its working directory
+                r = subprocess.run([path, "-d", str(device_index), "-vkfft", "0"], capture_output=True, text=True, timeout=900,
+                                   cwd=td)
             m = re.search(r"Benchmark score VkFFT: (\d+)", r.stdout)
             per = {mm.group(1): float(mm.group(2)) for mm in re.finditer(r"VkFFT System: (\d+) .*?avg_time_per_step: ([0-9.]+) ms", r.stdout)}
             out[key] = {"score": int(m.group(1)) if m else None, "rc": r.returncode, "seconds": round(time.time() - t0, 1),
@@ -496,6 +530,7 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE config 3-5 legs")
     ap.add_argument("--no-sample0", action="store_true", help="skip the reference's sample_0 benchmark binaries")
     ap.add_argument("--no-dist", action="store_true", help="skip the distributed 2^26 record (N >= 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy (rank 0)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -553,6 +588,7 @@ def main():
     for _ in range(args.warmup):
         sweep()
     barrier()
+    start = buf.clone() if args.dump_outputs and rank == 0 else None
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
@@ -572,6 +608,11 @@ def main():
         ms_step = float(t.item())
     fl_step = sum(flops_pair(n, pts) for n in ns)
     value = world * fl_step / (ms_step * 1e-3) / 1e9
+    dumped = None
+    if start is not None:
+        dumped = dump_outputs(args.dump_outputs, torch, vk, apps, lp, buf, start, args.steps, sweep)
+        del start
+        torch.cuda.empty_cache()
 
     # ---- per-N breakdown (rank 0 reports) ---------------------------------------------------------------------------
     peak, peak_src = measured_peaks()
@@ -737,6 +778,8 @@ def main():
     }
     if dist_rec is not None:
         line["dist_2p26"] = dist_rec
+    if dumped is not None:
+        line["dump_outputs"] = dumped
     if world == 1 and not args.no_cpu:
         line["cpu_baseline"], _ = cpu_baseline()
     else:

@@ -1,14 +1,19 @@
 """CPU: the C-ABI library loads, exports every symbol include/b200fft.h declares, the header-only vkFFT.h shim
 compiles as C and C++ with the reference's struct layout, and host-side error behaviour matches the reference.
 (No compute calls here: there is no GPU in the -m "not gpu" environment.)"""
+import json
 import os
 import re
 import subprocess
+import sys
 import tempfile
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# sizeof / offsetof of every member of the drop-in structs as the reference's own vkFFT.h (VkFFT 1.3.4, VKFFT_BACKEND=1)
+# lays them out; written by `python tests/test_abi.py <reference>/vkFFT`
+REFERENCE_LAYOUT = os.path.join(ROOT, "tests", "golden", "reference_vkfft_layout.json")
 
 
 def test_library_exports_every_declared_symbol(built_lib):
@@ -92,23 +97,25 @@ def _layout_dump(include_dirs, defines, members, lang):
 def test_vkfft_shim_header_layout(lang):
     """sizeof/offsetof of the drop-in structs == the reference's VKFFT_BACKEND==1 build.  The probe is compiled, RUN and
     compared: against the known numbers of the reference headers (SURVEY.md section 7: VkFFTConfiguration 1168 B,
-    VkFFTLaunchParams 80 B, buffer@152, numberBatches@272, doublePrecision@360, performR2C@408) and -- when the reference
-    tree is present -- member by member against a probe compiled from the reference's own header."""
+    VkFFTLaunchParams 80 B, buffer@152, numberBatches@272, doublePrecision@360, performR2C@408) and member by member against
+    the same probe compiled from the reference's own header (REFERENCE_LAYOUT)."""
     cuda = "/usr/local/cuda"
     if not os.path.exists(os.path.join(cuda, "include", "cuda.h")):
         pytest.skip("CUDA headers not present")
-    hdr = open(os.path.join(ROOT, "include", "vkFFT.h")).read()
-    members = {"VkFFTConfiguration": _struct_members(hdr, "VkFFTConfiguration"),
-               "VkFFTLaunchParams": _struct_members(hdr, "VkFFTLaunchParams")}
+    members = _shim_members()
     assert len(members["VkFFTConfiguration"]) > 100 and len(members["VkFFTLaunchParams"]) >= 9
     mine = _layout_dump([os.path.join(ROOT, "include")], ["VKFFT_BACKEND=1"], members, lang)
     assert mine["sizeof.VkFFTConfiguration"] == 1168 and mine["sizeof.VkFFTLaunchParams"] == 80
     assert mine["VkFFTConfiguration.buffer"] == 152 and mine["VkFFTConfiguration.numberBatches"] == 272
     assert mine["VkFFTConfiguration.doublePrecision"] == 360 and mine["VkFFTConfiguration.performR2C"] == 408
-    ref_inc = "/root/reference/vkFFT"
-    if lang == "c++" and os.path.exists(os.path.join(ref_inc, "vkFFT.h")):
-        theirs = _layout_dump([ref_inc], ["VKFFT_BACKEND=1"], members, lang)
-        assert mine == theirs, {k: (mine[k], theirs.get(k)) for k in mine if mine[k] != theirs.get(k)}
+    theirs = json.load(open(REFERENCE_LAYOUT))
+    assert mine == theirs, {k: (mine[k], theirs.get(k)) for k in mine if mine[k] != theirs.get(k)}
+
+
+def _shim_members():
+    hdr = open(os.path.join(ROOT, "include", "vkFFT.h")).read()
+    return {"VkFFTConfiguration": _struct_members(hdr, "VkFFTConfiguration"),
+            "VkFFTLaunchParams": _struct_members(hdr, "VkFFTLaunchParams")}
 
 
 def test_python_api_host_side_errors(built_lib):
@@ -166,3 +173,10 @@ def test_reference_testsuite_sources_build_against_the_shim(built_lib):
     for s in ("b200fft_plan_create", "b200fft_exec", "b200fft_plan_destroy", "b200fft_plan_axis_uploads"):
         assert s in syms, s                      # the samples' initializeVkFFT / VkFFTAppend / deleteVkFFT end in the C ABI
     assert "nvrtcCompileProgram" not in syms     # nothing is JIT-compiled any more
+
+
+if __name__ == "__main__":
+    # regenerate REFERENCE_LAYOUT from the directory holding the reference's vkFFT.h
+    with open(REFERENCE_LAYOUT, "w") as f:
+        json.dump(_layout_dump([sys.argv[1]], ["VKFFT_BACKEND=1"], _shim_members(), "c++"), f, indent=0, sort_keys=True)
+        f.write("\n")

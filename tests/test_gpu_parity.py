@@ -199,7 +199,7 @@ def test_r2c_c2r(gpu, shape, batch, double):
 @pytest.mark.parametrize("inverse", [-1, 1])
 def test_dct(gpu, kind, shape, batch, double, inverse):
     import vkfft_b200 as vk
-    from gpu_util import assert_f32_parity, ref_inplace
+    from gpu_util import assert_f32_parity
     rdt = np.float64 if double else np.float32
     x = orc.random_input((batch,) + tuple(reversed(shape)), rdt, seed=kind + sum(shape))
     cfg = vk.VkFFTConfiguration(FFTdim=len(shape), size=list(shape), numberBatches=batch, device=0, performDCT=kind,
@@ -209,7 +209,7 @@ def test_dct(gpu, kind, shape, batch, double, inverse):
     if double:
         assert orc.error_metrics(y, ref)["l2_rel"] < TOL64
     else:
-        assert_f32_parity(y, ref, lambda: ref_inplace(x, shape, batch, inverse, perform_dct=kind))
+        assert_f32_parity(y, ref, x, shape, batch, inverse, perform_dct=kind)
 
 
 def test_out_of_place_formatted_buffers(gpu):
@@ -253,7 +253,7 @@ def test_out_of_place_formatted_buffers(gpu):
 @pytest.mark.parametrize("inverse", [-1, 1])
 def test_dst(gpu, kind, shape, batch, double, inverse):
     import vkfft_b200 as vk
-    from gpu_util import assert_f32_parity, ref_inplace
+    from gpu_util import assert_f32_parity
     rdt = np.float64 if double else np.float32
     x = orc.random_input((batch,) + tuple(reversed(shape)), rdt, seed=kind + sum(shape))
     cfg = vk.VkFFTConfiguration(FFTdim=len(shape), size=list(shape), numberBatches=batch, device=0, performDST=kind,
@@ -263,7 +263,7 @@ def test_dst(gpu, kind, shape, batch, double, inverse):
     if double:
         assert orc.error_metrics(y, ref)["l2_rel"] < TOL64
     else:
-        assert_f32_parity(y, ref, lambda: ref_inplace(x, shape, batch, inverse, perform_dst=kind))
+        assert_f32_parity(y, ref, x, shape, batch, inverse, perform_dst=kind)
 
 
 @pytest.mark.parametrize("shape,batch,double", [((1 << 20,), 3, False), ((2 * 4391,), 4, False), ((1 << 17, 4), 1, True)])

@@ -207,5 +207,5 @@ def test_dct_2_and_3_lengths_without_ahead_of_time_kernels(gpu, shape, batch, do
     if double:
         assert orc.error_metrics(got, ref)["l2_rel"] < 1e-12
     else:      # 1e-6, or -- where the transform's conditioning puts both engines beyond it -- at least as close as the reference
-        from gpu_util import assert_f32_parity, ref_inplace
-        assert_f32_parity(got, ref, lambda: ref_inplace(x, shape, batch, -1, perform_dct=kind))
+        from gpu_util import assert_f32_parity
+        assert_f32_parity(got, ref, x, shape, batch, -1, perform_dct=kind)
